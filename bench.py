@@ -2,7 +2,7 @@
 """Benchmark of the hot path: one full training step (fwd + loss + bwd + Adam) of the 3-layer GCN student with
 logit-KD on the ARXIV-shape synthetic graph (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (see README/DESIGN.md for the keys).  metric = edges aggregated per second,
 edges/s = 2 * L * nnz(Â) / t_step  (L=3 aggregations forward + 3 backward, nnz of the matrix the SpMM walks).
@@ -314,6 +314,12 @@ def run_single(args):
     ms_step = e0.elapsed_time(e1) / args.steps
     clocks = clk.summary()
     losses = tr.loss_out.tolist()
+    # what the last timed step returned (losses) and left behind (its logits, the parameters after its Adam update),
+    # copied before the later phases run further steps
+    outputs = None
+    if args.dump_outputs:
+        outputs = {"loss": tr.loss_out.cpu(), "logits": tr.Y[-1].cpu()}
+        outputs.update({k: v.cpu() for k, v in tr.state_dict().items()})
 
     # ---- phase 2: end to end — every step copies ITS inputs from pinned host memory and its losses are read back.
     # Two device input sets + two captured graphs: the upload of step k+1 (copy stream) overlaps the compute of step k.
@@ -423,7 +429,18 @@ def run_single(args):
                             "step (double-buffered, overlapping the previous step), 3 loss scalars read back"},
             "gpu_launches": launches * args.steps, "gpu_launches_per_step": launches,
             "clocks": clocks, "loss": losses}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     emit_json_line(line)
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """One float32 <name>.npy per array, so that two builds run with the same arguments can be compared output by output."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(d / f"{name}.npy", t.detach().float().numpy())
 
 
 def main():
@@ -435,10 +452,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the fp64 CPU parity leg (~20 s of host time)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's losses, logits and updated parameters "
+                         "as DIR/<name>.npy (float32, ~28 MB)")
     args = ap.parse_args()
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl == "reference" or world > 1 or args.gpus > 1):
+        ap.error("--dump-outputs is implemented for the single-GPU run of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
-    world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1 or args.gpus > 1:
         from efficient_gnns_b200 import dist_bench
         return dist_bench.run(args)
