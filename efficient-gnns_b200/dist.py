@@ -109,24 +109,29 @@ def scatter_rows(t: torch.Tensor, plan: ShardPlan, fill=0) -> torch.Tensor:
 class ShardedGCNTrainer(GCNStudentTrainer):
     """One rank of the node-parallel GCN student; same step semantics as GCNStudentTrainer."""
 
+    aux_loss_supported = False       # out_feat's gradient would need its own route through the row shards
+
     def __init__(self, adj: SparseTensor, dims: List[int], group=None, **kw):
         assert dist.is_initialized(), "torch.distributed must be initialised (backend nccl)"
         self.group = group
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
+        self.n_global = adj.size(0)
+        super().__init__(adj, dims, **kw)
+        dev = self.device
+        self.full = {k: torch.empty(self.plan.n_pad, k, device=dev) for k in set(dims[1:])}   # all-gather targets
+        self.sum_buf = {k: torch.empty(2, k, device=dev) for k in set(dims[1:])}
+        self.row0 = self.rank * self.plan.block
+
+    def _prepare_graph(self, adj: SparseTensor):
+        """This rank's rows of the relabelled Â (forward and, Â being symmetric, backward); buffers of the common block size."""
         norm = gcn_norm(adj)
         if not _is_symmetric(norm):
             raise NotImplementedError("node-parallel backward relies on a symmetric normalised adjacency")
         self.plan = make_plan(norm.storage.rowcount(), self.world)
         rel = relabel_adjacency(norm, self.plan)
         rowptr, col, val = shard_rows(rel, self.plan, self.rank)
-        self._shard = csr_graph_from(rowptr, col, val, self.plan.real_rows(self.rank), self.plan.n_pad)
-        self.n_global = adj.size(0)
-        super().__init__(adj, dims, _prebuilt_graph=self._shard, _rows_alloc=self.plan.block, **kw)
-        dev = self.device
-        self.full = {k: torch.empty(self.plan.n_pad, k, device=dev) for k in set(dims[1:])}   # all-gather targets
-        self.sum_buf = {k: torch.empty(2, k, device=dev) for k in set(dims[1:])}
-        self.row0 = self.rank * self.plan.block
-        self.n_train_global = 0
+        shard = csr_graph_from(rowptr, col, val, self.plan.real_rows(self.rank), self.plan.n_pad)
+        return shard, shard, self.plan.block
 
     # -- data placement helpers (original node order -> this rank's block)
     def shard_inputs(self, x, y, train_idx, teacher_logits=None):
@@ -199,9 +204,7 @@ class ShardedGCNTrainer(GCNStudentTrainer):
                 ops.affine_relu_dropout(self.Y[l], self.bn[l][2], self.bn[l][3], True, self.p, self.seed, l, out=self.A[l],
                                         step_dev=self.step_count, step_mul=self.L, row_offset=r0)
             else:
-                scale = self.gamma[l] * torch.rsqrt(self.running_var[l] + self.bn_eps)
-                shift = self.beta[l] - self.running_mean[l] * scale
-                ops.affine_relu_dropout(self.Y[l], scale, shift, True, 0.0, out=self.A[l])
+                ops.affine_relu_dropout(self.Y[l], *self._bn_eval(l), True, 0.0, out=self.A[l])
             inp = self.A[l]
         return self.Y[-1]
 
@@ -232,14 +235,8 @@ class ShardedGCNTrainer(GCNStudentTrainer):
                     self.ggamma[l - 1].zero_(); self.gbeta[l - 1].zero_()
         self._wgrad_join()
 
-    def _step_impl(self, x_pad, y_loc, train_loc, teacher_loc):
-        logits = self.forward(x_pad, training=True)
-        self.dY[-1].zero_()
-        ops.kd_loss_fwd_bwd(logits, y_loc, train_loc, teacher_loc, self.alpha, self.kd_T, d_logits=self.dY[-1],
-                            loss_out=self.loss_out, partial=self.kd_part, n_norm=self.n_train_global)
-        self.backward(x_pad)
+    def _reduce_grads(self):
         dist.all_reduce(self._grads_buf, group=self.group)      # gradients + the three loss scalars
-        ops.adam_step(self.params, self.grads, self.exp_avg, self.exp_avg_sq, self.step_count, self.lr)
 
     def exchange_bytes_per_step(self) -> int:
         """Bytes each rank RECEIVES over NVLink per step in the all-gathers (the data-path collectives)."""

@@ -13,136 +13,74 @@ backward:
 
 No autograd tape, no torch BatchNorm / Adam, no cuBLAS on the step where the tensor-core tilings apply (round 1 ran SAGE
 through the module path: 25 % of its step was torch BN/elementwise and 12 % cuBLAS fallbacks).  ``train_step(..., aux=)`` adds
-an auxiliary distillation loss on ``out_feat`` exactly as engine.GCNStudentTrainer does (kd + beta*aux; configs[2] = G-CRD).
+an auxiliary distillation loss on ``out_feat`` as every engine.StudentTrainer does (kd + beta*aux; configs[2] = G-CRD).
 Parameters use nn.Linear's [out, in] layout and the reference module's state_dict keys (convs.i.lin_l.weight / .bias,
 convs.i.lin_r.weight, bns.i.*).
 """
 from __future__ import annotations
 
 import math
-from typing import Dict, List, Optional
+from typing import List, Optional, Tuple
 
 import torch
 
 from . import lib, ops
+from .engine import StudentTrainer
 from .sparse import CsrGraph, SparseTensor
 
 
-class SAGEStudentTrainer:
+class SAGEStudentTrainer(StudentTrainer):
+    views = ("Wl", "bl", "Wr", "gamma", "beta")
+
     def __init__(self, adj: SparseTensor, dims: List[int], dropout: float = 0.5, lr: float = 0.01, seed: int = 0,
                  alpha: float = 0.9, kd_T: float = 4.0, bn_eps: float = 1e-5, bn_momentum: float = 0.1,
                  fuse_row_passes: bool = True):
         assert adj.is_cuda(), "the engine runs on a CUDA device"
         for d in dims:
             assert d % 4 == 0 and d <= 1024, "layer widths must be multiples of 4 (128-bit rows)"
-        self.device = dev = adj.device
-        self.dims, self.L = list(dims), len(dims) - 1
-        self.p, self.lr, self.alpha, self.kd_T = float(dropout), float(lr), float(alpha), float(kd_T)
-        self.bn_eps, self.bn_momentum, self.seed = bn_eps, bn_momentum, int(seed)
-        self.N = N = adj.size(0)
         st = adj.set_value(None).storage                      # SAGEConv drops edge values (A.3)
         self.G: CsrGraph = st.engine_csr_unweighted()         # mean over in-neighbours
         self.Gt: CsrGraph = st.engine_csc("mean")             # transpose with 1/deg(dst) weights: the mean's backward
         self.nnz = self.G.nnz
-        sizes = []
-        for l in range(self.L):
-            sizes += [dims[l + 1] * dims[l], dims[l + 1], dims[l + 1] * dims[l]]      # W_l [out,in], b_l, W_r [out,in]
-            if l < self.L - 1:
-                sizes += [dims[l + 1], dims[l + 1]]
-        n_par = sum(sizes)
-        self.params = torch.zeros(n_par, device=dev)
-        self.n_par_pad = (n_par + 3) // 4 * 4
-        self._grads_buf = torch.zeros(self.n_par_pad + 4, device=dev)
-        self.grads = self._grads_buf[:n_par]
-        self.loss_out = self._grads_buf[self.n_par_pad:self.n_par_pad + 3]
-        self.exp_avg, self.exp_avg_sq = torch.zeros(n_par, device=dev), torch.zeros(n_par, device=dev)
-        self.step_count = torch.zeros(1, dtype=torch.int32, device=dev)
-        self.Wl, self.bl, self.Wr, self.gamma, self.beta = [], [], [], [], []
-        self.gWl, self.gbl, self.gWr, self.ggamma, self.gbeta = [], [], [], [], []
-        off = 0
-
-        def take(n, shape):
-            nonlocal off
-            v = (self.params[off:off + n].view(shape), self.grads[off:off + n].view(shape))
-            off += n
-            return v
-        for l in range(self.L):
-            a, b = take(dims[l + 1] * dims[l], (dims[l + 1], dims[l])); self.Wl.append(a); self.gWl.append(b)
-            a, b = take(dims[l + 1], (dims[l + 1],)); self.bl.append(a); self.gbl.append(b)
-            a, b = take(dims[l + 1] * dims[l], (dims[l + 1], dims[l])); self.Wr.append(a); self.gWr.append(b)
-            if l < self.L - 1:
-                a, b = take(dims[l + 1], (dims[l + 1],)); self.gamma.append(a); self.ggamma.append(b)
-                a, b = take(dims[l + 1], (dims[l + 1],)); self.beta.append(a); self.gbeta.append(b)
-        self.running_mean = [torch.zeros(d, device=dev) for d in dims[1:-1]]
-        self.running_var = [torch.ones(d, device=dev) for d in dims[1:-1]]
+        super().__init__(adj.device, dims, adj.size(0), dropout, lr, seed, alpha, kd_T, bn_eps, bn_momentum)
+        dev, N, L = self.device, self.N, self.L
         buf = lambda k: torch.zeros(N, k, device=dev)
-        self.M = [buf(dims[l]) for l in range(self.L)]                 # mean-aggregated input of layer l
-        self.Y = [buf(dims[l + 1]) for l in range(self.L)]
-        self.A = [buf(dims[l + 1]) for l in range(self.L - 1)]
-        self.dY = [buf(dims[l + 1]) for l in range(self.L)]
-        self.dM = [buf(dims[l]) for l in range(self.L)]
-        self.dA = [buf(dims[l + 1]) for l in range(self.L - 1)]
-        self.bn = [torch.empty(4, dims[l + 1], device=dev) for l in range(self.L - 1)]
-        self.rs = ops.rows_slots(N)
+        self.M = [buf(dims[l]) for l in range(L)]                 # mean-aggregated input of layer l
+        self.Y = [buf(dims[l + 1]) for l in range(L)]
+        self.A = [buf(dims[l + 1]) for l in range(L - 1)]
+        self.dY = [buf(dims[l + 1]) for l in range(L)]
+        self.dM = [buf(dims[l]) for l in range(L)]
+        self.dA = [buf(dims[l + 1]) for l in range(L - 1)]
+        self.bn = [torch.empty(4, dims[l + 1], device=dev) for l in range(L - 1)]
         # BatchNorm statistics / backward reductions taken in GEMM epilogues (engine.py, SURVEY §8 f1)
         self._gemm_part = {k: torch.empty(ops.gemm_stat_slots(N, k), 2, k, device=dev)
                            for k in set(self.dims[1:-1]) if fuse_row_passes and ops.gemm_stats_supported(k)}
-        self._static: Dict[str, torch.Tensor] = {}
-        self.kd_part = torch.empty(2 * int(lib.load().b200gnn_kd_partials(N)), device=dev)
         self.split = {}
-        wg = [(dims[l], dims[l + 1]) for l in range(self.L) if ops.wgrad_supported(dims[l], dims[l + 1])]
-        self.wgrad_ws = torch.empty(148 * max(a * ((b + 31) // 32 * 32) for a, b in wg), device=dev) if wg else None
-        self.loss_aux = None
-        self._graph = None
-        self.reset_parameters(seed)
+        self.wgrad_ws = self._wgrad_workspace()
 
     # ------------------------------------------------------------------ parameters
-    def reset_parameters(self, seed: int = 0):
-        """nn.Linear.reset_parameters (kaiming-uniform(a=sqrt 5) => U(+-1/sqrt(fan_in)) for weight and bias), BN ones/zeros."""
-        g = torch.Generator().manual_seed(seed)
+    @staticmethod
+    def param_table(dims: List[int]) -> List[Tuple[str, Tuple[int, ...], str]]:
+        """Keys of the reference's SAGE module: per layer convs.i.lin_l.weight [out,in] (nn.Linear's layout) and bias,
+        convs.i.lin_r.weight [out,in]; per hidden layer bns.i.weight / bias."""
+        table = []
+        for l in range(len(dims) - 1):
+            w = (dims[l + 1], dims[l])
+            table += [(f"convs.{l}.lin_l.weight", w, "Wl"), (f"convs.{l}.lin_l.bias", (dims[l + 1],), "bl"),
+                      (f"convs.{l}.lin_r.weight", w, "Wr")]
+            if l < len(dims) - 2:
+                table += StudentTrainer._bn_table(l, dims[l + 1])
+        return table
+
+    def _init_weights(self, g: torch.Generator):
+        """nn.Linear.reset_parameters: kaiming-uniform(a=sqrt 5) => U(+-1/sqrt(fan_in)) for weight and bias."""
         for l in range(self.L):
             bound = 1.0 / math.sqrt(self.dims[l])
             self.Wl[l].copy_((torch.rand(self.dims[l + 1], self.dims[l], generator=g) * 2 - 1) * bound)
             self.bl[l].copy_((torch.rand(self.dims[l + 1], generator=g) * 2 - 1) * bound)
             self.Wr[l].copy_((torch.rand(self.dims[l + 1], self.dims[l], generator=g) * 2 - 1) * bound)
-        for l in range(self.L - 1):
-            self.gamma[l].fill_(1.0); self.beta[l].zero_()
-            self.running_mean[l].zero_(); self.running_var[l].fill_(1.0)
-        self.exp_avg.zero_(); self.exp_avg_sq.zero_(); self.step_count.zero_()
-
-    def state_dict(self) -> Dict[str, torch.Tensor]:
-        sd = {}
-        for l in range(self.L):
-            sd[f"convs.{l}.lin_l.weight"] = self.Wl[l].detach().clone()
-            sd[f"convs.{l}.lin_l.bias"] = self.bl[l].detach().clone()
-            sd[f"convs.{l}.lin_r.weight"] = self.Wr[l].detach().clone()
-        for l in range(self.L - 1):
-            sd[f"bns.{l}.weight"] = self.gamma[l].detach().clone()
-            sd[f"bns.{l}.bias"] = self.beta[l].detach().clone()
-            sd[f"bns.{l}.running_mean"] = self.running_mean[l].clone()
-            sd[f"bns.{l}.running_var"] = self.running_var[l].clone()
-        return sd
-
-    def load_state_dict(self, sd):
-        for l in range(self.L):
-            self.Wl[l].copy_(sd[f"convs.{l}.lin_l.weight"]); self.bl[l].copy_(sd[f"convs.{l}.lin_l.bias"])
-            self.Wr[l].copy_(sd[f"convs.{l}.lin_r.weight"])
-        for l in range(self.L - 1):
-            self.gamma[l].copy_(sd[f"bns.{l}.weight"]); self.beta[l].copy_(sd[f"bns.{l}.bias"])
 
     # ------------------------------------------------------------------ helpers
-    def _part(self, k):
-        key = f"part{k}"
-        if key not in self._static:
-            self._static[key] = torch.empty(self.rs, 2, k, device=self.device)
-        return self._static[key]
-
-    def _coef(self, k):
-        key = f"coef{k}"
-        if key not in self._static:
-            self._static[key] = torch.empty(3, k, device=self.device)
-        return self._static[key]
-
     def _split(self, w: torch.Tensor, transpose: bool, key: str):
         shape = (w.shape[1], w.shape[0]) if transpose else tuple(w.shape)
         if key not in self.split:
@@ -162,12 +100,6 @@ class SAGEStudentTrainer:
             torch.mm(x.t(), g, out=tmp)
         lib.check(lib.load().b200gnn_transpose_f32(lib.dptr(tmp, torch.float32, "tmp"), k_in, n_out,
                                                    lib.dptr(out_t, torch.float32, "out"), lib.stream_ptr()), "transpose_f32")
-
-    def out_feat(self) -> torch.Tensor:
-        return self.A[-1]
-
-    def dropout_offset(self, layer: int, step: int) -> int:
-        return layer + step * self.L
 
     # ------------------------------------------------------------------ forward / backward
     def forward(self, x: torch.Tensor, training: bool = True) -> torch.Tensor:
@@ -192,9 +124,7 @@ class SAGEStudentTrainer:
                 ops.affine_relu_dropout(self.Y[l], self.bn[l][2], self.bn[l][3], True, self.p, self.seed, l, out=self.A[l],
                                         step_dev=self.step_count, step_mul=self.L)
             else:
-                scale = self.gamma[l] * torch.rsqrt(self.running_var[l] + self.bn_eps)
-                shift = self.beta[l] - self.running_mean[l] * scale
-                ops.affine_relu_dropout(self.Y[l], scale, shift, True, 0.0, out=self.A[l])
+                ops.affine_relu_dropout(self.Y[l], *self._bn_eval(l), True, 0.0, out=self.A[l])
             inp = self.A[l]
         return self.Y[-1]
 
@@ -230,50 +160,3 @@ class SAGEStudentTrainer:
             ops.bn_act_bwd(d_prev, self.A[l - 1], self.Y[l - 1], self.bn[l - 1][0], self.bn[l - 1][1], self.gamma[l - 1], self.p,
                            d_y=self.dY[l - 1], d_gamma=self.ggamma[l - 1], d_beta=self.gbeta[l - 1], partial=self._part(kp),
                            coef=self._coef(kp), want_dbias=False)
-
-    def _loss(self, x, y, train_idx, teacher_logits):
-        logits = self.forward(x, training=True)
-        self.dY[-1].zero_()
-        ops.kd_loss_fwd_bwd(logits, y, train_idx, teacher_logits, self.alpha, self.kd_T, d_logits=self.dY[-1],
-                            loss_out=self.loss_out, partial=self.kd_part)
-
-    def _step_impl(self, x, y, train_idx, teacher_logits):
-        self._loss(x, y, train_idx, teacher_logits)
-        self.backward(x)
-        ops.adam_step(self.params, self.grads, self.exp_avg, self.exp_avg_sq, self.step_count, self.lr)
-
-    def train_step(self, x, y, train_idx, teacher_logits=None, aux=None, beta: float = 1.0) -> torch.Tensor:
-        """One reference ``train()`` call for ``--gnn sage``: supervised / kd, or kd + beta*aux with ``aux(out_feat)`` as in
-        engine.GCNStudentTrainer.train_step.  Returns the device tensor [loss, loss_cls, loss_kd]."""
-        if aux is None:
-            self._step_impl(x, y, train_idx, teacher_logits)
-            return self.loss_out
-        self._loss(x, y, train_idx, teacher_logits)
-        feat = self.out_feat().detach().requires_grad_(True)
-        with torch.enable_grad():
-            loss_aux = aux(feat)
-            (loss_aux * beta).backward()
-        d_feat = feat.grad if feat.grad is not None else torch.zeros_like(feat)
-        self.backward(x, d_out_feat=d_feat)
-        ops.adam_step(self.params, self.grads, self.exp_avg, self.exp_avg_sq, self.step_count, self.lr)
-        self.loss_aux = loss_aux.detach()
-        self.loss_out[0].add_(self.loss_aux * beta)
-        return self.loss_out
-
-    # ------------------------------------------------------------------ CUDA graph
-    def capture(self, x, y, train_idx, teacher_logits=None, warmup: int = 2):
-        s = torch.cuda.Stream()
-        s.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(s):
-            for _ in range(warmup):
-                self._step_impl(x, y, train_idx, teacher_logits)
-        torch.cuda.current_stream().wait_stream(s)
-        torch.cuda.synchronize()
-        self._graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self._graph):
-            self._step_impl(x, y, train_idx, teacher_logits)
-        return self
-
-    def replay(self) -> torch.Tensor:
-        self._graph.replay()
-        return self.loss_out

@@ -213,6 +213,8 @@ def _numel(shape) -> int:
 class HybridGCNTrainer(GCNStudentTrainer):
     """One rank of the hybrid-layout GCN student; same step semantics as GCNStudentTrainer (engine.py)."""
 
+    aux_loss_supported = False       # out_feat's gradient would need its own route through the R / C layouts
+
     def __init__(self, adj: SparseTensor, dims: List[int], group=None, exchange: str = "peer", _fake=None, fuse_r2c: bool = True,
                  fuse_c2r: bool = True, fuse_gather: bool = False, **kw):
         self.group = group
@@ -227,18 +229,8 @@ class HybridGCNTrainer(GCNStudentTrainer):
             assert dist.is_initialized(), "torch.distributed must be initialised"
             self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
         P = self.world
-        norm = gcn_norm(adj)
-        if not _is_symmetric(norm):
-            raise NotImplementedError("the multi-GPU backward relies on a symmetric normalised adjacency")
-        self.plan = make_dense_plan(norm.storage.rowcount(), P)
-        rel = relabel(norm, self.plan)
-        rowptr, col, val = row_shard(rel, self.plan, self.rank)
-        self.n_p = self.plan.counts[self.rank]
         self.n_global = adj.size(0)
-        self._shard = csr_graph_from(rowptr, col, val, self.n_p, self.n_global)
-        frp, fcol, fval = rel.csr()
-        self.Gfull = csr_graph_from(frp, fcol, fval, self.n_global, self.n_global)
-        super().__init__(adj, dims, _prebuilt_graph=self._shard, _rows_alloc=self.plan.block, **kw)
+        super().__init__(adj, dims, **kw)
         dev = self.device
         N, L = self.n_global, self.L
         self.row0 = self.plan.offsets[self.rank]
@@ -296,7 +288,21 @@ class HybridGCNTrainer(GCNStudentTrainer):
                             for l in range(L - 1) if self.col_mode[dims[l + 1]]}
         self.rs_full = ops.rows_slots(N)
         self._layer_in: List[Optional[torch.Tensor]] = [None] * L
-        self.n_train_global = 0
+
+    def _prepare_graph(self, adj: SparseTensor):
+        """This rank's rows of the relabelled Â for the row-sharded aggregations (forward and, Â being symmetric, backward),
+        buffers of the common block size; the whole relabelled Â (self.Gfull) for the feature-parallel ones."""
+        norm = gcn_norm(adj)
+        if not _is_symmetric(norm):
+            raise NotImplementedError("the multi-GPU backward relies on a symmetric normalised adjacency")
+        self.plan = make_dense_plan(norm.storage.rowcount(), self.world)
+        rel = relabel(norm, self.plan)
+        rowptr, col, val = row_shard(rel, self.plan, self.rank)
+        self.n_p = self.plan.counts[self.rank]
+        shard = csr_graph_from(rowptr, col, val, self.n_p, self.n_global)
+        frp, fcol, fval = rel.csr()
+        self.Gfull = csr_graph_from(frp, fcol, fval, self.n_global, self.n_global)
+        return shard, shard, self.plan.block
 
     # ------------------------------------------------------------------ data placement
     def shard_inputs(self, x, y, train_idx, teacher_logits=None):
@@ -385,7 +391,7 @@ class HybridGCNTrainer(GCNStudentTrainer):
                                     self.running_mean[0], self.running_var[0], out=self.bn[0])
                     self._act_R(0, self.Y[0], self.bn[0], self.A[0], True)
                 else:
-                    self._eval_act(0, self.Y[0], self.A[0])
+                    ops.affine_relu_dropout(self.Y[0], *self._bn_eval(0), True, 0.0, out=self.A[0])
                 inp = self.A[0]
                 continue
             src = x_in if l == 0 else inp
@@ -430,9 +436,8 @@ class HybridGCNTrainer(GCNStudentTrainer):
                                                    rowmap=self.rowmap_full, k_global=k, col_offset=self.rank * kc)
                 else:
                     ops.spmm_csr(self.Gfull, c[f"Hc{l}"], "sum", bias=bias_c, out=c[f"Yc{l}"])
-                    scale = self._cols(self.gamma[l], k) * torch.rsqrt(self._cols(self.running_var[l], k) + self.bn_eps)
-                    shift = self._cols(self.beta[l], k) - self._cols(self.running_mean[l], k) * scale
-                    ops.affine_relu_dropout(c[f"Yc{l}"], scale, shift, True, 0.0, out=c[f"Ac{l}"])
+                    cols = slice(self.rank * kc, (self.rank + 1) * kc)
+                    ops.affine_relu_dropout(c[f"Yc{l}"], *self._bn_eval(l, cols), True, 0.0, out=c[f"Ac{l}"])
                 self.ex.c2r(c[f"Ac{l}"], c[f"A_R{l}"], f"A_R{l}")
                 inp = c[f"A_R{l}"]
             else:
@@ -450,7 +455,7 @@ class HybridGCNTrainer(GCNStudentTrainer):
                     self._act_R(l, self.Y[l], self.bn[l], self.A[l], True)
                 else:
                     ops.spmm_csr(self.G, c[f"Hfull{l}"], "sum", bias=self.b[l], out=self.Y[l])
-                    self._eval_act(l, self.Y[l], self.A[l])
+                    ops.affine_relu_dropout(self.Y[l], *self._bn_eval(l), True, 0.0, out=self.A[l])
                 inp = self.A[l]
         raise AssertionError("unreachable")
 
@@ -473,11 +478,6 @@ class HybridGCNTrainer(GCNStudentTrainer):
         hi, lo = ops.split_tf32(self.W[l], transpose=False, hi=self.W_split[l][0], lo=self.W_split[l][1])
         ops.gemm_tf32x3_scatter(d_out, hi, lo, self.ex.fused_r2c_targets(name), self.row0)
         self.ex.barrier()
-
-    def _eval_act(self, l: int, y: torch.Tensor, out: torch.Tensor):
-        scale = self.gamma[l] * torch.rsqrt(self.running_var[l] + self.bn_eps)
-        shift = self.beta[l] - self.running_mean[l] * scale
-        ops.affine_relu_dropout(y, scale, shift, True, 0.0, out=out)
 
     def logits_rows(self) -> torch.Tensor:
         l = self.L - 1
@@ -576,17 +576,11 @@ class HybridGCNTrainer(GCNStudentTrainer):
         return self._static[key]
 
     # ------------------------------------------------------------------ step
-    def _step_impl(self, x_in, y_loc, train_loc, teacher_loc):
-        logits = self.forward(x_in, training=True)
-        self.dY[-1].zero_()
-        ops.kd_loss_fwd_bwd(logits, y_loc, train_loc, teacher_loc, self.alpha, self.kd_T, d_logits=self.dY[-1],
-                            loss_out=self.loss_out, partial=self.kd_part, n_norm=self.n_train_global)
-        self.backward(x_in)
+    def _reduce_grads(self):
         # gradients and loss scalars (one buffer): every rank's contribution lands in every rank's [P, n] block and is summed
         # in rank order (fp64) -> bit-identical replicas, no all-reduce
         self.ex.allgather_vec(self._grads_buf, self.grads_all, "grads_all")
         ops.partial_reduce(self.grads_all, out=self._grads_buf)
-        ops.adam_step(self.params, self.grads, self.exp_avg, self.exp_avg_sq, self.step_count, self.lr)
 
     def exchange_bytes_per_step(self) -> int:
         """Bytes each rank RECEIVES over NVLink per training step (data-path exchanges only)."""
