@@ -9,7 +9,7 @@ Layout
   nn.py        GCNConv / SAGEConv / MessagePassing mirrors of the PyG surface
   criterion.py fused distillation criteria (same names/arguments as the reference's criterion.py)
   engine.py    graph-captured full training step for the benchmark configs
-  engine_sage.py / rgcn.py     fused GraphSAGE step, full-batch R-GCN inference
+  engine_sage.py / rgcn.py     fused GraphSAGE step; fused R-GCN training step and full-batch R-GCN inference
   hybrid.py / peer.py / hybrid_gat.py   multi-GPU: node-parallel dense ops + feature-parallel aggregations, peer-memory exchange
   dist.py      round-1 node-parallel engine (all-gather per aggregation), kept as the baseline
   sampling.py  device-side GraphSAINT random-walk sampler, small-graph DataLoader

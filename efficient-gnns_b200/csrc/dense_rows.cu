@@ -395,6 +395,16 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const 
 }
 __global__ void adam_tick_kernel(int32_t* step) { *step += 1; }
 
+// dY = dOut * [Xout > 0] * inv_keep over n_vec float4s (Xout = dropout(relu(Y)) > 0 <=> ReLU-active and kept)
+__global__ void __launch_bounds__(256) relu_dropout_bwd_kernel(const float4* dOut, const float4* __restrict__ Xout,
+                                                               int64_t n_vec, float inv_keep, float4* dY) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_vec; i += (int64_t)gridDim.x * blockDim.x) {
+    const float4 d = dOut[i], x = __ldg(Xout + i);
+    dY[i] = make_float4(x.x > 0.f ? d.x * inv_keep : 0.f, x.y > 0.f ? d.y * inv_keep : 0.f,
+                        x.z > 0.f ? d.z * inv_keep : 0.f, x.w > 0.f ? d.w * inv_keep : 0.f);
+  }
+}
+
 static inline int grid_for(int64_t n_items, int per_cta, int cap = 148 * 8) {
   int64_t g = (n_items + per_cta - 1) / per_cta;
   if (g > cap) g = cap;
@@ -526,6 +536,19 @@ extern "C" int b200gnn_dropout_mask_u8(uint8_t* mask, int64_t n_rows, int64_t K,
   uint32_t thr16 = 0;
   const int p16 = dropout_p16(p, thr16) ? 1 : 0;
   dropout_mask_kernel<<<grid_for(n_vec, 256 * 4), 256, 0, (cudaStream_t)stream>>>(mask, n_vec, p, p16, thr16, seed, offset);
+  return check_launch();
+}
+
+extern "C" int b200gnn_relu_dropout_bwd_f32(const float* dOut, const float* Xout, int64_t n_rows, int64_t K, float p, float* dY,
+                                            void* stream) {
+  if (!rows_ok(n_rows, K) || !dOut || !Xout || !dY || p < 0.f || p >= 1.f || !aligned_to(dOut, 16) || !aligned_to(Xout, 16) ||
+      !aligned_to(dY, 16))
+    return B200GNN_ERR_BAD_ARG;
+  if (n_rows == 0) return B200GNN_OK;
+  const int64_t n_vec = n_rows * (K / 4);
+  const float inv_keep = p > 0.f ? 1.f / (1.f - p) : 1.f;
+  relu_dropout_bwd_kernel<<<grid_for(n_vec, 256 * 4), 256, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const float4*>(dOut), reinterpret_cast<const float4*>(Xout), n_vec, inv_keep, reinterpret_cast<float4*>(dY));
   return check_launch();
 }
 

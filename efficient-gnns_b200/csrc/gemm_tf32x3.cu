@@ -461,6 +461,266 @@ static int launch(const float* A, int64_t lda, const float* B_hi, const float* B
   return check_launch();
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Grouped form: G row ranges of one A / C pair, each with its own B (and K, bias), in one launch — the per-node-type
+// weights of an R-GCN layer.  Same pipeline as gemm_tf32x3_kernel with the plain / bias / accumulate epilogue only; the
+// tile scheduler maps a tile to (group, m-tile, n-tile) through the prefix table tile0, so no tile straddles two groups
+// and each group's tiles do exactly the arithmetic a launch of the plain kernel on that group would do.  A group with
+// K = 0 has no MMAs: its tiles store the bias alone (the caller leaves such groups out in accumulate mode).
+// The tensor maps travel in the kernel parameters (~6.6 KB, large kernel parameters), so a launch needs no upload and
+// captures into a CUDA graph.
+constexpr int MAX_GROUPS = 16;
+
+struct GroupMaps { CUtensorMap a, bhi, blo; };
+
+struct GroupedParams {
+  GroupMaps map[MAX_GROUPS];
+  const float* bias[MAX_GROUPS];
+  int64_t row0[MAX_GROUPS];
+  int32_t rows[MAX_GROUPS], K[MAX_GROUPS];
+  int32_t tile0[MAX_GROUPS + 1];          // first tile of each group; tile0[n_groups] = total tiles
+  float* C;
+  int64_t ldc;
+  int32_t N, n_groups, accumulate;
+};
+
+template <class C>
+__global__ void __launch_bounds__(THREADS, 1) gemm_grouped_kernel(const __grid_constant__ GroupedParams p) {
+  constexpr int BN = C::BN, STAGES = C::STAGES, STAGE_BYTES = C::STAGE_BYTES, B_TILE_BYTES = C::B_TILE_BYTES;
+  constexpr int TMEM_COLS = C::TMEM_COLS, ACC_STRIDE = C::ACC_STRIDE, ACC_HALF = C::ACC_HALF;
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + STAGES * STAGE_BYTES);
+  uint64_t* full = bars;
+  uint64_t* split = bars + STAGES;
+  uint64_t* empty = bars + 2 * STAGES;
+  uint64_t* acc_full = bars + 3 * STAGES;
+  uint64_t* acc_empty = acc_full + ACC_STAGES;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + ACC_STAGES);
+  float* epi_smem = reinterpret_cast<float*>(smem + STAGES * STAGE_BYTES + BAR_BYTES);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&split[s], 128); mbar_init(&empty[s], 1); }
+    for (int a = 0; a < ACC_STAGES; ++a) { mbar_init(&acc_full[a], 1); mbar_init(&acc_empty[a], 128); }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 2) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
+                 "n"(TMEM_COLS));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+
+  const int num_n = (p.N + BN - 1) / BN;
+  const int num_tiles = p.tile0[p.n_groups];
+  // tile -> (group, first row inside the group, first column)
+  auto locate = [&](int tile, int& g, int& m0, int& n0) {
+    g = 0;
+    while (tile >= p.tile0[g + 1]) ++g;
+    const int lt = tile - p.tile0[g];
+    m0 = (lt / num_n) * BM;
+    n0 = (lt % num_n) * BN;
+  };
+
+  if (warp == 0) {
+    // ------------------------------------------------------------------ TMA producer
+    if (lane == 0) {
+      int s = 0; uint32_t ph = 0;
+      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
+        int g, m0, n0;
+        locate(tile, g, m0, n0);
+        const int num_kb = (p.K[g] + BK - 1) / BK;
+        for (int kb = 0; kb < num_kb; ++kb) {
+          mbar_wait(&empty[s], ph ^ 1);
+          uint8_t* st = smem + s * STAGE_BYTES;
+          mbar_expect_tx(&full[s], TILE_BYTES + 2 * B_TILE_BYTES);
+          tma_load_2d(&p.map[g].a, &full[s], st, kb * BK, m0);
+          tma_load_2d(&p.map[g].bhi, &full[s], st + 2 * TILE_BYTES, kb * BK, n0);
+          tma_load_2d(&p.map[g].blo, &full[s], st + 2 * TILE_BYTES + B_TILE_BYTES, kb * BK, n0);
+          if (++s == STAGES) { s = 0; ph ^= 1; }
+        }
+      }
+    }
+  } else if (warp == 1) {
+    // ------------------------------------------------------------------ MMA issuer
+    if (lane == 0) {
+      const uint32_t idesc = make_idesc<BN>();
+      int s = 0; uint32_t ph = 0; int a = 0; uint32_t aph = 0;
+      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
+        int g, m0, n0;
+        locate(tile, g, m0, n0);
+        const int num_kb = (p.K[g] + BK - 1) / BK;
+        if (num_kb == 0) continue;                     // bias-only tile: no accumulator
+        mbar_wait(&acc_empty[a], aph ^ 1);
+        tc_fence_after();
+        const uint32_t d_tmem = tmem_base + (uint32_t)(a * ACC_STRIDE);
+        for (int kb = 0; kb < num_kb; ++kb) {
+          mbar_wait(&full[s], ph);
+          mbar_wait(&split[s], ph);
+          tc_fence_after();
+          const uint32_t st = smem_u32(smem + s * STAGE_BYTES);
+#pragma unroll
+          for (int k = 0; k < BK / UMMA_K; ++k) {
+            const uint32_t koff = k * UMMA_K * 4;
+            const uint64_t a_hi = make_smem_desc(st + koff), a_lo = make_smem_desc(st + TILE_BYTES + koff);
+            const uint64_t b_hi = make_smem_desc(st + 2 * TILE_BYTES + koff);
+            const uint64_t b_lo = make_smem_desc(st + 2 * TILE_BYTES + B_TILE_BYTES + koff);
+            mma_tf32(d_tmem + ACC_HALF, a_lo, b_hi, idesc, (kb | k) != 0);
+            mma_tf32(d_tmem + ACC_HALF, a_hi, b_lo, idesc, 1);
+            mma_tf32(d_tmem, a_hi, b_hi, idesc, (kb | k) != 0);
+          }
+          mma_commit(&empty[s]);
+          if (++s == STAGES) { s = 0; ph ^= 1; }
+        }
+        mma_commit(&acc_full[a]);
+        if (++a == ACC_STAGES) { a = 0; aph ^= 1; }
+      }
+    }
+  } else if (warp >= 4 && warp < 8) {
+    // ------------------------------------------------------------------ splitter: A -> (A_hi, A_lo)
+    const int t = threadIdx.x - 128;
+    int s = 0; uint32_t ph = 0;
+    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
+      int g, m0, n0;
+      locate(tile, g, m0, n0);
+      const int num_kb = (p.K[g] + BK - 1) / BK;
+      for (int kb = 0; kb < num_kb; ++kb) {
+        mbar_wait(&full[s], ph);
+        uint4* hi = reinterpret_cast<uint4*>(smem + s * STAGE_BYTES);
+        uint4* lo = reinterpret_cast<uint4*>(smem + s * STAGE_BYTES + TILE_BYTES);
+#pragma unroll
+        for (int i = 0; i < TILE_BYTES / 16 / 128; ++i) {
+          const int o = i * 128 + t;
+          const uint4 v = hi[o];
+          uint4 h, l;
+          split4(v, h, l);
+          hi[o] = h;
+          lo[o] = l;
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        mbar_arrive(&split[s]);
+        if (++s == STAGES) { s = 0; ph ^= 1; }
+      }
+    }
+  } else if (warp >= 8) {
+    // ------------------------------------------------------------------ epilogue (plain / bias / accumulate)
+    const int q = warp & 3;
+    int a = 0; uint32_t aph = 0;
+    const bool vec_ok = (p.ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0);
+    constexpr int NCHUNK = (BN + 31) / 32;
+    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
+      int g, m0, n0;
+      locate(tile, g, m0, n0);
+      const bool mma = p.K[g] > 0;
+      const int M = p.rows[g];
+      const float* bias = p.bias[g];
+      float* Cg = p.C + p.row0[g] * p.ldc;
+      const int row = m0 + q * 32 + lane;
+#pragma unroll 1
+      for (int c = 0; c < NCHUNK; ++c) {
+        uint32_t r[32];
+        if (mma) {
+          if (c == 0) {
+            mbar_wait(&acc_full[a], aph);
+            tc_fence_after();
+          }
+          uint32_t rc[32];
+          tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(a * ACC_STRIDE + c * 32), r);
+          tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(a * ACC_STRIDE + ACC_HALF + c * 32), rc);
+#pragma unroll
+          for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(__uint_as_float(r[j]) + __uint_as_float(rc[j]));
+        } else {
+#pragma unroll
+          for (int j = 0; j < 32; ++j) r[j] = 0u;
+        }
+        const int col0 = n0 + c * 32;
+        if (vec_ok && col0 + 32 <= p.N) {
+          float* tl = epi_smem + (warp - 8) * (32 * EPI_LD);
+#pragma unroll
+          for (int j = 0; j < 32; j += 4)
+            *reinterpret_cast<float4*>(tl + lane * EPI_LD + j) =
+                make_float4(__uint_as_float(r[j]), __uint_as_float(r[j + 1]), __uint_as_float(r[j + 2]), __uint_as_float(r[j + 3]));
+          __syncwarp();
+          const int sub = lane >> 3, cq = (lane & 7) * 4;
+          float4 b4 = make_float4(0.f, 0.f, 0.f, 0.f);
+          if (bias) b4 = make_float4(__ldg(bias + col0 + cq), __ldg(bias + col0 + cq + 1), __ldg(bias + col0 + cq + 2),
+                                     __ldg(bias + col0 + cq + 3));
+#pragma unroll
+          for (int it = 0; it < 8; ++it) {
+            const int rr = it * 4 + sub;
+            const int grow = m0 + q * 32 + rr;
+            float4 v = *reinterpret_cast<const float4*>(tl + rr * EPI_LD + cq);
+            v.x += b4.x; v.y += b4.y; v.z += b4.z; v.w += b4.w;
+            if (grow < M) {
+              float4* dst = reinterpret_cast<float4*>(Cg + (size_t)grow * p.ldc + col0 + cq);
+              if (p.accumulate) { const float4 o = *dst; v.x += o.x; v.y += o.y; v.z += o.z; v.w += o.w; }
+              *dst = v;
+            }
+          }
+          __syncwarp();
+        } else if (row < M && col0 < p.N) {
+          float* dst = Cg + (size_t)row * p.ldc + col0;
+#pragma unroll
+          for (int j = 0; j < 32; ++j)
+            if (col0 + j < p.N) dst[j] = __uint_as_float(r[j]) + (bias ? __ldg(bias + col0 + j) : 0.f) + (p.accumulate ? dst[j] : 0.f);
+        }
+      }
+      if (mma) {
+        tc_fence_before();
+        mbar_arrive(&acc_empty[a]);
+        if (++a == ACC_STAGES) { a = 0; aph ^= 1; }
+      }
+    }
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS));
+  }
+}
+
+template <class C>
+static int launch_grouped(const float* A, int64_t lda, const b200gnn_gemm_group* groups, int32_t n_groups, GroupedParams& p,
+                          cudaStream_t stream) {
+  const int num_n = (p.N + C::BN - 1) / C::BN;
+  int64_t tiles = 0;
+  int ng = 0;
+  for (int i = 0; i < n_groups; ++i) {
+    const b200gnn_gemm_group& gr = groups[i];
+    if (gr.rows == 0 || (gr.K == 0 && p.accumulate)) continue;     // nothing to store
+    if (gr.K > 0 && (!make_map(&p.map[ng].a, A + gr.row0 * lda, gr.rows, gr.K, lda, BM) ||
+                     !make_map(&p.map[ng].bhi, gr.B_hi, p.N, gr.K, gr.ldb, C::BN) ||
+                     !make_map(&p.map[ng].blo, gr.B_lo, p.N, gr.K, gr.ldb, C::BN)))
+      return B200GNN_ERR_UNSUPPORTED;
+    p.bias[ng] = gr.bias; p.row0[ng] = gr.row0; p.rows[ng] = (int32_t)gr.rows; p.K[ng] = (int32_t)gr.K;
+    p.tile0[ng] = (int32_t)tiles;
+    tiles += ((gr.rows + BM - 1) / BM) * num_n;
+    ++ng;
+  }
+  if (tiles >= INT32_MAX) return B200GNN_ERR_BAD_ARG;
+  p.n_groups = ng;
+  p.tile0[ng] = (int32_t)tiles;
+  if (tiles == 0) return B200GNN_OK;
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  static bool attr_set[64] = {};
+  if (dev >= 0 && dev < 64 && !attr_set[dev]) {
+    cudaError_t e = cudaFuncSetAttribute(gemm_grouped_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
+    if (e != cudaSuccess) { set_cuda_error(e); return B200GNN_ERR_CUDA; }
+    attr_set[dev] = true;
+  }
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int grid = tiles < sms ? (int)tiles : sms;
+  gemm_grouped_kernel<C><<<grid, THREADS, C::SMEM_BYTES, stream>>>(p);
+  return check_launch();
+}
+
 }  // namespace gemm
 }  // namespace b200gnn
 
@@ -554,6 +814,26 @@ extern "C" int b200gnn_gemm_tf32x3_f32(const float* A, int64_t lda, const float*
 extern "C" int b200gnn_gemm_tf32x3_acc_f32(const float* A, int64_t lda, const float* B_hi, const float* B_lo, int64_t ldb,
                                            float* C, int64_t ldc, int64_t M, int64_t N, int64_t K, void* stream) {
   return gemm_dispatch(A, lda, B_hi, B_lo, ldb, C, ldc, M, N, K, nullptr, 1, stream);
+}
+
+// C[row0_g + m, :N] (+)= A[row0_g + m, :K_g] · B_g^T (+ bias_g) for every group g, one launch (see gemm_grouped_kernel).
+extern "C" int b200gnn_gemm_tf32x3_grouped_f32(const float* A, int64_t lda, float* C, int64_t ldc, int64_t N,
+                                               const b200gnn_gemm_group* groups, int32_t n_groups, int accumulate,
+                                               void* stream) {
+  if (!A || !C || !groups || n_groups < 0 || n_groups > gemm::MAX_GROUPS || N <= 0 || N >= INT32_MAX || ldc < N || lda <= 0)
+    return B200GNN_ERR_BAD_ARG;
+  for (int i = 0; i < n_groups; ++i) {
+    const b200gnn_gemm_group& g = groups[i];
+    if (g.row0 < 0 || g.rows < 0 || g.rows >= INT32_MAX || g.K < 0 || g.K > lda || g.K >= INT32_MAX)
+      return B200GNN_ERR_BAD_ARG;
+    if (g.K > 0 && (!g.B_hi || !g.B_lo || g.ldb < g.K)) return B200GNN_ERR_BAD_ARG;
+    if (g.K % 4 || (g.K > 0 && (g.ldb % 4 || !aligned_to(g.B_hi, 16) || !aligned_to(g.B_lo, 16)))) return B200GNN_ERR_UNSUPPORTED;
+  }
+  if (lda % 4 || !aligned_to(A, 16)) return B200GNN_ERR_UNSUPPORTED;
+  gemm::GroupedParams p{};
+  p.C = C; p.ldc = ldc; p.N = (int32_t)N; p.accumulate = accumulate ? 1 : 0;
+  if (N <= 48) return gemm::launch_grouped<gemm::Cfg<48, 4>>(A, lda, groups, n_groups, p, (cudaStream_t)stream);
+  return gemm::launch_grouped<gemm::Cfg<128, 3>>(A, lda, groups, n_groups, p, (cudaStream_t)stream);
 }
 
 // C = A · B^T (+bias) with the output SCATTERED BY COLUMN BLOCK to `world` destination buffers: columns [q*kc, (q+1)*kc)

@@ -56,6 +56,7 @@ SIGNATURES = {
     "b200gnn_affine_relu_dropout_scatter_f32": (_int, [_f32p, _f32p, _i64, _i64, _f32p, _f32p, _int, _f32, _u64, _u64,
                                                        _i32p, _u64, _i32p, _u64, _i64, _i64, _ptr, _ptr, _i32, _i64, _ptr]),
     "b200gnn_dropout_mask_u8": (_int, [_ptr, _i64, _i64, _f32, _u64, _u64, _ptr]),
+    "b200gnn_relu_dropout_bwd_f32": (_int, [_f32p, _f32p, _i64, _i64, _f32, _f32p, _ptr]),
     "b200gnn_bn_act_bwd_f32": (_int, [_f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _i64, _i64, _f32, _f32p, _f32p,
                                       _f32p, _f32p, _f32p, _i64, _f32p, _ptr]),
     "b200gnn_bn_act_bwd_reduce_f32": (_int, [_f32p, _f32p, _f32p, _f32p, _f32p, _i64, _i64, _f32, _f32p, _i64, _ptr]),
@@ -78,6 +79,7 @@ SIGNATURES = {
     "b200gnn_gemm_tf32x3_bnbwd_f32": (_int, [_f32p, _i64, _f32p, _f32p, _i64, _f32p, _i64, _i64, _i64, _i64, _int,
                                              _f32p, _f32p, _f32p, _f32p, _f32, _f32p, _i64, _ptr]),
     "b200gnn_gemm_tf32x3_acc_f32": (_int, [_f32p, _i64, _f32p, _f32p, _i64, _f32p, _i64, _i64, _i64, _i64, _ptr]),
+    "b200gnn_gemm_tf32x3_grouped_f32": (_int, [_f32p, _i64, _f32p, _i64, _i64, _ptr, _i32, _int, _ptr]),
     "b200gnn_gemm_tf32x3_scatter_f32": (_int, [_f32p, _i64, _f32p, _f32p, _i64, _ptr, _i32, _i64, _i64, _i64, _i64, _f32p, _ptr]),
     "b200gnn_gemm_tf32x3_bcast_f32": (_int, [_f32p, _i64, _f32p, _f32p, _i64, _ptr, _i32, _i64, _i64, _i64, _i64, _i64, _f32p, _ptr]),
     "b200gnn_wgrad_workspace_floats": (_i64, [_i64, _i64]),
@@ -127,6 +129,13 @@ SIGNATURES = {
 class Copy2D(C.Structure):
     """struct b200gnn_copy2d (include/b200gnn.h)."""
     _fields_ = [("dst", C.c_void_p), ("src", C.c_void_p), ("ld_dst", C.c_int64), ("ld_src", C.c_int64), ("rows", C.c_int64)]
+
+
+class GemmGroup(C.Structure):
+    """struct b200gnn_gemm_group (include/b200gnn.h)."""
+    _fields_ = [("B_hi", C.c_void_p), ("B_lo", C.c_void_p), ("ldb", C.c_int64), ("bias", C.c_void_p), ("row0", C.c_int64),
+                ("rows", C.c_int64), ("K", C.c_int64)]
+
 
 _lib = None
 

@@ -119,6 +119,17 @@ def _f32(t, name):
     return lib.dptr(t, torch.float32, name)
 
 
+def _f32_rows(t, name):
+    """Device pointer of a row-strided fp32 matrix view (unit column stride; the row pitch is passed separately)."""
+    if t is None:
+        return None
+    if t.dim() != 2 or (t.stride(1) != 1 and t.shape[1] > 1):
+        raise lib.B200GnnError(f"{name}: expected a 2-D view with unit column stride")
+    if not t.is_cuda or t.dtype != torch.float32:
+        raise lib.B200GnnError(f"{name}: expected a CUDA float32 tensor (got {t.device}, {t.dtype}); there is no CPU fallback")
+    return t.data_ptr()
+
+
 def rows_slots(n_rows: int) -> int:
     return int(lib.load().b200gnn_rows_slots(n_rows))
 
@@ -201,6 +212,15 @@ def affine_relu_dropout_scatter(y: torch.Tensor, scale, shift, relu: bool, p: fl
     return out
 
 
+def relu_dropout_bwd(d_out: torch.Tensor, x_out: torch.Tensor, p: float, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Backward of x_out = dropout_p(relu(y)): d_y = d_out * [x_out > 0] / (1-p); ``out`` may be ``d_out``."""
+    n, K = x_out.shape
+    out = torch.empty_like(x_out) if out is None else out
+    lib.check(lib.load().b200gnn_relu_dropout_bwd_f32(_f32(d_out, "d_out"), _f32(x_out, "x_out"), n, K, float(p),
+                                                      _f32(out, "out"), lib.stream_ptr()), "relu_dropout_bwd_f32")
+    return out
+
+
 def dropout_mask(n_rows: int, K: int, p: float, seed: int, offset: int, device="cuda") -> torch.Tensor:
     """The keep-mask (uint8 [n,K]) that affine_relu_dropout uses for (seed, offset)."""
     mask = torch.empty(n_rows, K, dtype=torch.uint8, device=device)
@@ -239,7 +259,8 @@ def adam_step(params, grads, exp_avg, exp_avg_sq, step: torch.Tensor, lr: float,
 
 def kd_loss_fwd_bwd(logits, labels, train_idx, teacher_logits=None, alpha: float = 0.9, T: float = 4.0,
                     d_logits=None, loss_out=None, partial=None, n_norm: int = 0):
-    """Fused CE / logit-KD over rows train_idx of FULL [N,C] matrices; returns (loss_out[3], d_logits [N,C])."""
+    """Fused CE / logit-KD over rows train_idx of FULL [N,C] matrices (row-strided views accepted, e.g. the first C columns
+    of a padded buffer); returns (loss_out[3], d_logits [N,C])."""
     N, C = logits.shape
     n_train = train_idx.numel() if train_idx is not None else N
     L = lib.load()
@@ -250,9 +271,9 @@ def kd_loss_fwd_bwd(logits, labels, train_idx, teacher_logits=None, alpha: float
     if partial is None:
         partial = torch.empty(2 * int(L.b200gnn_kd_partials(max(n_train, 1))), dtype=torch.float32, device=logits.device)
     lib.check(L.b200gnn_kd_loss_fwd_bwd_f32(
-        _f32(logits, "logits"), logits.stride(0), lib.dptr(train_idx, torch.int64, "train_idx"), n_train,
-        lib.dptr(labels, torch.int64, "labels"), _f32(teacher_logits, "teacher_logits"),
-        teacher_logits.stride(0) if teacher_logits is not None else 0, C, alpha, T, n_norm, _f32(d_logits, "d_logits"),
+        _f32_rows(logits, "logits"), logits.stride(0), lib.dptr(train_idx, torch.int64, "train_idx"), n_train,
+        lib.dptr(labels, torch.int64, "labels"), _f32_rows(teacher_logits, "teacher_logits"),
+        teacher_logits.stride(0) if teacher_logits is not None else 0, C, alpha, T, n_norm, _f32_rows(d_logits, "d_logits"),
         d_logits.stride(0), _f32(loss_out, "loss_out"), _f32(partial, "partial"), lib.stream_ptr()), "kd_loss_fwd_bwd_f32")
     return loss_out, d_logits
 
@@ -272,7 +293,8 @@ def split_tf32(w: torch.Tensor, transpose: bool = False, hi: Optional[torch.Tens
 
 def gemm_tf32x3(a: torch.Tensor, b_hi: torch.Tensor, b_lo: torch.Tensor, bias: Optional[torch.Tensor] = None,
                 out: Optional[torch.Tensor] = None, accumulate: bool = False) -> torch.Tensor:
-    """out[M,N] (+)= a[M,K] @ b[N,K]^T (+bias) with fp32 fidelity on the tensor cores (b pre-split by split_tf32)."""
+    """out[M,N] (+)= a[M,K] @ b[N,K]^T (+bias) with fp32 fidelity on the tensor cores (b pre-split by split_tf32); a and out
+    may be row-strided views."""
     M, K = a.shape
     N = b_hi.shape[0]
     assert b_hi.shape == b_lo.shape and b_hi.shape[1] == K
@@ -282,13 +304,31 @@ def gemm_tf32x3(a: torch.Tensor, b_hi: torch.Tensor, b_lo: torch.Tensor, bias: O
     L = lib.load()
     if accumulate:
         assert bias is None
-        lib.check(L.b200gnn_gemm_tf32x3_acc_f32(_f32(a, "a"), a.stride(0), _f32(b_hi, "b_hi"), _f32(b_lo, "b_lo"),
-                                                b_hi.stride(0), _f32(out, "out"), out.stride(0), M, N, K, lib.stream_ptr()),
+        lib.check(L.b200gnn_gemm_tf32x3_acc_f32(_f32_rows(a, "a"), a.stride(0), _f32(b_hi, "b_hi"), _f32(b_lo, "b_lo"),
+                                                b_hi.stride(0), _f32_rows(out, "out"), out.stride(0), M, N, K, lib.stream_ptr()),
                   "gemm_tf32x3_acc_f32")
         return out
-    lib.check(L.b200gnn_gemm_tf32x3_f32(_f32(a, "a"), a.stride(0), _f32(b_hi, "b_hi"), _f32(b_lo, "b_lo"),
-                                        b_hi.stride(0), _f32(out, "out"), out.stride(0), M, N, K,
+    lib.check(L.b200gnn_gemm_tf32x3_f32(_f32_rows(a, "a"), a.stride(0), _f32(b_hi, "b_hi"), _f32(b_lo, "b_lo"),
+                                        b_hi.stride(0), _f32_rows(out, "out"), out.stride(0), M, N, K,
                                         _f32(bias, "bias"), lib.stream_ptr()), "gemm_tf32x3_f32")
+    return out
+
+
+def gemm_tf32x3_grouped(a: torch.Tensor, out: torch.Tensor, groups, accumulate: bool = False) -> torch.Tensor:
+    """One launch of out[r0:r0+m, :N] (+)= a[r0:r0+m, :K_g] @ b_g[N, K_g]^T (+bias_g) over the groups
+    ``(row0, rows, b_hi, b_lo, bias)`` (b pre-split by split_tf32, K_g = b_hi.shape[1], bias may be None; b_hi None means
+    K_g = 0).  ``a`` and ``out`` may be row-strided views (unit column stride)."""
+    N = out.shape[1]
+    arr = (lib.GemmGroup * max(len(groups), 1))()
+    for i, (row0, rows, b_hi, b_lo, bias) in enumerate(groups):
+        if b_hi is not None:
+            assert b_hi.shape == b_lo.shape and b_hi.shape[0] == N and b_hi.stride(0) == b_lo.stride(0)
+            arr[i].B_hi, arr[i].B_lo, arr[i].ldb, arr[i].K = _f32_rows(b_hi, "b_hi"), _f32_rows(b_lo, "b_lo"), b_hi.stride(0), b_hi.shape[1]
+        arr[i].bias = _f32(bias, "bias")
+        arr[i].row0, arr[i].rows = int(row0), int(rows)
+    lib.check(lib.load().b200gnn_gemm_tf32x3_grouped_f32(_f32_rows(a, "a"), a.stride(0), _f32_rows(out, "out"), out.stride(0), N,
+                                                         arr, len(groups), int(accumulate), lib.stream_ptr()),
+              "gemm_tf32x3_grouped_f32")
     return out
 
 
@@ -362,7 +402,8 @@ def wgrad_supported(k_in: int, n_out: int) -> bool:
 
 def gemm_wgrad_tf32x3(x: torch.Tensor, g: torch.Tensor, out: Optional[torch.Tensor] = None,
                       workspace: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """out[Kin,Nout] = x[Nn,Kin]^T @ g[Nn,Nout] on the tensor cores with fp32 fidelity (split-K over nodes)."""
+    """out[Kin,Nout] = x[Nn,Kin]^T @ g[Nn,Nout] on the tensor cores with fp32 fidelity (split-K over nodes); x and g may be
+    row-strided views."""
     nn_, k_in = x.shape
     n_out = g.shape[1]
     assert g.shape[0] == nn_
@@ -371,7 +412,7 @@ def gemm_wgrad_tf32x3(x: torch.Tensor, g: torch.Tensor, out: Optional[torch.Tens
         out = torch.empty(k_in, n_out, dtype=torch.float32, device=x.device)
     if workspace is None:
         workspace = torch.empty(int(L.b200gnn_wgrad_workspace_floats(k_in, n_out)), dtype=torch.float32, device=x.device)
-    lib.check(L.b200gnn_gemm_wgrad_tf32x3_f32(_f32(x, "x"), x.stride(0), _f32(g, "g"), g.stride(0), _f32(out, "out"), nn_,
+    lib.check(L.b200gnn_gemm_wgrad_tf32x3_f32(_f32_rows(x, "x"), x.stride(0), _f32_rows(g, "g"), g.stride(0), _f32(out, "out"), nn_,
                                               k_in, n_out, _f32(workspace, "workspace"), lib.stream_ptr()),
               "gemm_wgrad_tf32x3_f32")
     return out

@@ -187,6 +187,10 @@ int b200gnn_affine_relu_dropout_scatter_f32(const float* Y, float* out, int64_t 
                                             const int32_t* row_off, int32_t world, int64_t ld_dst, void* stream);
 int b200gnn_dropout_mask_u8(uint8_t* mask, int64_t n_rows, int64_t K, float p,
                             uint64_t seed, uint64_t offset, void* stream);
+/* Backward of out = dropout_p(relu(Y)) (no normalisation, the R-GCN hidden layers, mag_pyg/gnn.py:134-135):
+ * dY = dOut * [out > 0] / (1-p).  dY may alias dOut. */
+int b200gnn_relu_dropout_bwd_f32(const float* dOut, const float* Xout, int64_t n_rows, int64_t K, float p, float* dY,
+                                 void* stream);
 /* Backward of out = dropout_p(relu(BN_train(Y))): given dOut, out (for the
  * mask: out>0 <=> kept and active), Y and the saved batch mean/invstd, writes
  * dY, dgamma[K], dbeta[K] and (if non-NULL) dbias[K] = column sums of dY.
@@ -270,6 +274,21 @@ int b200gnn_gemm_tf32x3_f32(const float* A, int64_t lda, const float* B_hi,
 int b200gnn_gemm_tf32x3_acc_f32(const float* A, int64_t lda, const float* B_hi, const float* B_lo,
                                 int64_t ldb, float* C, int64_t ldc, int64_t M, int64_t N, int64_t K,
                                 void* stream);
+/* Grouped form over row ranges (the per-node-type weights of an R-GCN layer, mag_pyg/gnn.py:54-65), one launch:
+ *   C[row0_g + m, :N] (+)= A[row0_g + m, :K_g] * B_g[N, K_g]^T (+ bias_g[N])   for m < rows_g, every group g.
+ * A (pitch lda) and C (pitch ldc) are shared; each group brings its own pre-split B pair (pitch ldb), K_g (a multiple
+ * of 4, <= lda) and optional bias.  Groups must not overlap in C.  rows_g = 0 is a no-op; K_g = 0 stores the bias alone
+ * (zero without one), or leaves C unchanged when accumulating.  At most 16 groups.  Each group's tiles do the arithmetic
+ * of b200gnn_gemm_tf32x3_f32 / _acc_f32 on that group, bit for bit. */
+typedef struct b200gnn_gemm_group {
+  const float* B_hi;
+  const float* B_lo;
+  int64_t ldb;
+  const float* bias;
+  int64_t row0, rows, K;
+} b200gnn_gemm_group;
+int b200gnn_gemm_tf32x3_grouped_f32(const float* A, int64_t lda, float* C, int64_t ldc, int64_t N,
+                                    const b200gnn_gemm_group* groups, int32_t n_groups, int accumulate, void* stream);
 /* Row passes fused into the GEMM epilogue (SURVEY §8 f1; the reference runs conv -> BatchNorm1d -> ReLU -> dropout as
  * separate full-matrix ops, arxiv_pyg/gnn.py:47-50, and autograd walks them again backwards).  Each epilogue warp keeps
  * running column sums over the tiles of its CTA and stores them once: partial[slots][2][N], slots >=
