@@ -405,6 +405,24 @@ __global__ void __launch_bounds__(256) relu_dropout_bwd_kernel(const float4* dOu
   }
 }
 
+// The same with an added upstream gradient: dY = (dOut + dExtra) * [Xout > 0] * inv_keep, add then scale.  dExtra is an
+// unpadded row-strided [n, K_extra] matrix (scalar loads: its rows need not be 16-byte aligned); columns at or past
+// K_extra add 0.
+__global__ void __launch_bounds__(256) relu_dropout_bwd_add_kernel(const float4* dOut, const float* __restrict__ dExtra,
+                                                                   int64_t ld_extra, int64_t K_extra,
+                                                                   const float4* __restrict__ Xout, int64_t n_vec,
+                                                                   int64_t K_vec, float inv_keep, float4* dY) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_vec; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t row = i / K_vec, c = (i - row * K_vec) * 4;
+    const float* e = dExtra + row * ld_extra;
+    const float4 d = dOut[i], x = __ldg(Xout + i);
+    const float s0 = d.x + (c + 0 < K_extra ? __ldg(e + c + 0) : 0.f), s1 = d.y + (c + 1 < K_extra ? __ldg(e + c + 1) : 0.f);
+    const float s2 = d.z + (c + 2 < K_extra ? __ldg(e + c + 2) : 0.f), s3 = d.w + (c + 3 < K_extra ? __ldg(e + c + 3) : 0.f);
+    dY[i] = make_float4(x.x > 0.f ? s0 * inv_keep : 0.f, x.y > 0.f ? s1 * inv_keep : 0.f,
+                        x.z > 0.f ? s2 * inv_keep : 0.f, x.w > 0.f ? s3 * inv_keep : 0.f);
+  }
+}
+
 static inline int grid_for(int64_t n_items, int per_cta, int cap = 148 * 8) {
   int64_t g = (n_items + per_cta - 1) / per_cta;
   if (g > cap) g = cap;
@@ -549,6 +567,20 @@ extern "C" int b200gnn_relu_dropout_bwd_f32(const float* dOut, const float* Xout
   const float inv_keep = p > 0.f ? 1.f / (1.f - p) : 1.f;
   relu_dropout_bwd_kernel<<<grid_for(n_vec, 256 * 4), 256, 0, (cudaStream_t)stream>>>(
       reinterpret_cast<const float4*>(dOut), reinterpret_cast<const float4*>(Xout), n_vec, inv_keep, reinterpret_cast<float4*>(dY));
+  return check_launch();
+}
+
+extern "C" int b200gnn_relu_dropout_bwd_add_f32(const float* dOut, const float* dExtra, int64_t ld_extra, int64_t K_extra,
+                                                const float* Xout, int64_t n_rows, int64_t K, float p, float* dY, void* stream) {
+  if (!rows_ok(n_rows, K) || p < 0.f || p >= 1.f || K_extra < 0 || K_extra > K || ld_extra < K_extra) return B200GNN_ERR_BAD_ARG;
+  if (n_rows == 0) return B200GNN_OK;                  // empty tensors may come with null pointers
+  if (!dOut || !Xout || !dY || (K_extra > 0 && !dExtra) || !aligned_to(dOut, 16) || !aligned_to(Xout, 16) || !aligned_to(dY, 16))
+    return B200GNN_ERR_BAD_ARG;
+  const int64_t n_vec = n_rows * (K / 4);
+  const float inv_keep = p > 0.f ? 1.f / (1.f - p) : 1.f;
+  relu_dropout_bwd_add_kernel<<<grid_for(n_vec, 256 * 4), 256, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const float4*>(dOut), dExtra, ld_extra, K_extra, reinterpret_cast<const float4*>(Xout), n_vec, K / 4,
+      inv_keep, reinterpret_cast<float4*>(dY));
   return check_launch();
 }
 

@@ -57,6 +57,7 @@ SIGNATURES = {
                                                        _i32p, _u64, _i32p, _u64, _i64, _i64, _ptr, _ptr, _i32, _i64, _ptr]),
     "b200gnn_dropout_mask_u8": (_int, [_ptr, _i64, _i64, _f32, _u64, _u64, _ptr]),
     "b200gnn_relu_dropout_bwd_f32": (_int, [_f32p, _f32p, _i64, _i64, _f32, _f32p, _ptr]),
+    "b200gnn_relu_dropout_bwd_add_f32": (_int, [_f32p, _f32p, _i64, _i64, _f32p, _i64, _i64, _f32, _f32p, _ptr]),
     "b200gnn_bn_act_bwd_f32": (_int, [_f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _i64, _i64, _f32, _f32p, _f32p,
                                       _f32p, _f32p, _f32p, _i64, _f32p, _ptr]),
     "b200gnn_bn_act_bwd_reduce_f32": (_int, [_f32p, _f32p, _f32p, _f32p, _f32p, _i64, _i64, _f32, _f32p, _i64, _ptr]),

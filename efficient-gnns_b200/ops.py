@@ -212,12 +212,22 @@ def affine_relu_dropout_scatter(y: torch.Tensor, scale, shift, relu: bool, p: fl
     return out
 
 
-def relu_dropout_bwd(d_out: torch.Tensor, x_out: torch.Tensor, p: float, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Backward of x_out = dropout_p(relu(y)): d_y = d_out * [x_out > 0] / (1-p); ``out`` may be ``d_out``."""
+def relu_dropout_bwd(d_out: torch.Tensor, x_out: torch.Tensor, p: float, out: Optional[torch.Tensor] = None,
+                     extra: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Backward of x_out = dropout_p(relu(y)): d_y = d_out * [x_out > 0] / (1-p); ``out`` may be ``d_out``.  With ``extra``
+    (a row-strided [n, K_extra] view, K_extra <= K, e.g. the gradient of a loss on the unpadded hidden activation) the
+    upstream gradient is d_out + extra (zero past K_extra), added before the scaling."""
     n, K = x_out.shape
     out = torch.empty_like(x_out) if out is None else out
-    lib.check(lib.load().b200gnn_relu_dropout_bwd_f32(_f32(d_out, "d_out"), _f32(x_out, "x_out"), n, K, float(p),
-                                                      _f32(out, "out"), lib.stream_ptr()), "relu_dropout_bwd_f32")
+    if extra is None:
+        lib.check(lib.load().b200gnn_relu_dropout_bwd_f32(_f32(d_out, "d_out"), _f32(x_out, "x_out"), n, K, float(p),
+                                                          _f32(out, "out"), lib.stream_ptr()), "relu_dropout_bwd_f32")
+        return out
+    if extra.dim() != 2 or extra.shape[0] != n:
+        raise lib.B200GnnError(f"relu_dropout_bwd: extra must be [{n}, K_extra], got {tuple(extra.shape)}")
+    lib.check(lib.load().b200gnn_relu_dropout_bwd_add_f32(_f32(d_out, "d_out"), _f32_rows(extra, "extra"), extra.stride(0),
+                                                          extra.shape[1], _f32(x_out, "x_out"), n, K, float(p),
+                                                          _f32(out, "out"), lib.stream_ptr()), "relu_dropout_bwd_add_f32")
     return out
 
 

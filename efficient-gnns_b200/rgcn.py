@@ -168,7 +168,7 @@ class _Graph:
 
 class RGCNTrainer:
     """Fused training step of the reference's R-GCN (``RGCN.forward`` mag_pyg/gnn.py:126-138, ``train()`` :174-268 for
-    ``--training supervised|kd``) on device tensors, aggregate-first:
+    ``--training supervised|kd``, and with ``train_step(aux=)`` the representation losses) on device tensors, aggregate-first:
 
         M_l[i, s]  = mean over the edges j -> i of the s-th relation into type(i) of x_l[j]     one SpMM per layer
         out_l[t]   = x_l[t] · root_lins[t]ᵀ + b_t                                               one grouped GEMM
@@ -258,6 +258,7 @@ class RGCNTrainer:
         self._xpad: Dict[int, Tuple[torch.Tensor, torch.Tensor]] = {}
         self._last_p = 0.0
         self._last_inputs = None
+        self.loss_aux: Optional[torch.Tensor] = None
         self.reset_parameters(seed)
 
     # ------------------------------------------------------------------ parameters
@@ -427,8 +428,9 @@ class RGCNTrainer:
         else:
             torch.mm(x.t(), g, out=out)
 
-    def _backward(self, G: _Graph):
-        """Consumes G.dOut[-1] (d loss / d logits, padded columns zero); fills self.grads."""
+    def _backward(self, G: _Graph, d_out_feat: Optional[torch.Tensor] = None):
+        """Consumes G.dOut[-1] (d loss / d logits, padded columns zero); fills self.grads.  ``d_out_feat`` [n, hidden] (row
+        pitch free) is a gradient w.r.t. ``out_feat()``, added at the last hidden layer's ReLU/dropout backward."""
         L = lib.load()
         n = G.n
         self.grads.zero_()
@@ -460,7 +462,8 @@ class RGCNTrainer:
             ops.spmm_csr(G.bwd, G.dM[l].view(n * self.S_max, fi), "sum", out=dX)
             ops.gemm_tf32x3_grouped(dO, dX, self._groups(G, [f"rootT{l}_{t}" for t in range(self.T)]), accumulate=True)
             if l > 0:
-                ops.relu_dropout_bwd(dX, G.X[l], self._last_p, out=dX)
+                extra = d_out_feat if l == self.L - 1 else None
+                ops.relu_dropout_bwd(dX, G.X[l], self._last_p, out=dX, extra=extra)
             else:
                 ptrs, rows = self._table_args(None, grads=True)
                 lib.check(L.b200gnn_typed_scatter_f32(dX.data_ptr(), dX.stride(0), G.key[2].data_ptr(), G.key[3].data_ptr(),
@@ -490,25 +493,60 @@ class RGCNTrainer:
         G.dOut[-1][:, :self.dims[-1]].copy_(d_logits)
         self._backward(G)
 
-    def _step(self, x_dict, edge_index, edge_type, node_type, local_node_idx, y, train_idx, teacher_logits):
+    def _step(self, x_dict, edge_index, edge_type, node_type, local_node_idx, y, train_idx, teacher_logits, aux=None,
+              beta: float = 1.0):
         G = self._prepare(edge_index, edge_type, node_type, local_node_idx)
         logits = self._forward(G, x_dict, training=True)
         G.dOut[-1].zero_()
         ops.kd_loss_fwd_bwd(logits, y, train_idx, teacher_logits, self.alpha, self.kd_T,
                             d_logits=G.dOut[-1][:, :self.dims[-1]], loss_out=self.loss_out, partial=G.kd_part)
-        self._backward(G)
+        d_feat = None
+        if aux is not None:
+            feat = self.out_feat().detach().requires_grad_(True)
+            with torch.enable_grad():
+                loss_aux = aux(feat)
+                if loss_aux.requires_grad:
+                    (loss_aux * beta).backward()
+            self.loss_aux = loss_aux.detach()
+            d_feat = feat.grad                        # None: the loss does not depend on out_feat, the plain backward
+            if d_feat is not None and d_feat.stride(-1) != 1:
+                d_feat = d_feat.contiguous()
+        self._backward(G, d_feat)
         ops.adam_step(self.params, self.grads, self.exp_avg, self.exp_avg_sq, self.step_count, self.lr)
+        if aux is not None:
+            self.loss_out[0].add_(self.loss_aux * beta)
 
     def train_step(self, x_dict, edge_index, edge_type, node_type, local_node_idx, y, train_idx,
-                   teacher_logits: Optional[torch.Tensor] = None) -> torch.Tensor:
+                   teacher_logits: Optional[torch.Tensor] = None, aux=None, beta: float = 1.0) -> torch.Tensor:
         """One step of the reference's ``train()`` loop body (mag_pyg/gnn.py:188-257): forward with dropout, cross-entropy
         (supervised) or ``kd_criterion`` against ``teacher_logits`` [n, out_channels] over the rows ``train_idx``, backward,
         Adam.  ``y``: labels per row ([n] or [n, 1], int64).  Returns the device tensor [loss, loss_cls, loss_kd]; no host
-        sync for the loss (preparing a new graph reads its type counts and hub plan once)."""
+        sync for the loss (preparing a new graph reads its type counts and hub plan once).
+
+        Representation distillation (``--training fitnet|at|lpw|gpw|nce``): ``aux(feat)`` receives ``out_feat()`` — the
+        last hidden activation after ReLU and dropout, [n, hidden], detached and requiring grad — and returns the
+        auxiliary loss, built with ``criterion.*`` and any torch-side projection heads.  Its gradient (autograd) times
+        ``beta`` joins the backward at the last hidden layer's ReLU/dropout backward, so the dropout mask applies to it as
+        in the reference; ``self.loss_aux`` holds its value and ``loss[0]`` includes ``beta * loss_aux``.  Without
+        ``teacher_logits`` this is mag_pyg/gnn.py's ``loss_cls + beta * aux`` (:204-251), with them the ``kd + beta * aux``
+        of mag_pyg/gnn_kd_and_aux.py (:204-271).  A loss that does not depend on ``feat`` runs the plain backward.  On MAG:
+
+        * teacher features: a teacher ``RGCNTrainer`` (e.g. 3 x 512) on the same batch, ``forward(..., training=False)``,
+          then ``out_feat()[train_idx]`` (clone it: the buffer is reused by the next forward);
+        * LSP edges: ``nn.subgraph(train_idx, batch.edge_index, relabel_nodes=True)[0]`` (gnn.py:237);
+        * GSP and G-CRD row samples: ``sampled_inds=``, or numpy's global RNG as the reference draws them;
+        * the ``student_proj`` / ``teacher_proj`` heads of fitnet and nce (Linear -> BatchNorm1d -> ReLU, proj_dim 128)
+          stay torch modules; put their parameters in the caller's torch Adam at the engine's learning rate.  Adam is
+          elementwise, so this equals the reference's single optimizer over model and heads.
+
+        ``aux`` needs a hidden layer (num_layers >= 2)."""
+        if aux is not None and self.L < 2:
+            raise lib.B200GnnError("RGCNTrainer: aux= needs a hidden layer (num_layers >= 2): there is no out_feat")
         x_dict = {int(k): v for k, v in x_dict.items()}
         y = y.reshape(-1).contiguous()
         train_idx = train_idx.contiguous()
-        self._last_inputs = (x_dict, edge_index, edge_type, node_type, local_node_idx, y, train_idx, teacher_logits)
+        self._last_inputs = (x_dict, edge_index, edge_type, node_type, local_node_idx, y, train_idx, teacher_logits, aux,
+                             float(beta))
         self._step(*self._last_inputs)
         return self.loss_out
 

@@ -191,6 +191,14 @@ int b200gnn_dropout_mask_u8(uint8_t* mask, int64_t n_rows, int64_t K, float p,
  * dY = dOut * [out > 0] / (1-p).  dY may alias dOut. */
 int b200gnn_relu_dropout_bwd_f32(const float* dOut, const float* Xout, int64_t n_rows, int64_t K, float p, float* dY,
                                  void* stream);
+/* The same with an upstream gradient added before the ReLU/dropout backward: the reference's ``model.out_feat`` is the last
+ * hidden activation after ReLU and dropout (mag_pyg/gnn.py:133-136), so a loss on it joins the gradient coming back from
+ * the logits layer there.  dY[i, c] = (dOut[i, c] + (c < K_extra ? dExtra[i * ld_extra + c] : 0)) * [Xout[i, c] > 0] / (1-p),
+ * added, then scaled: bit-identical to b200gnn_relu_dropout_bwd_f32 on dOut + dExtra zero-padded to K columns.  dOut, Xout,
+ * dY: [n_rows, K] (K a multiple of 4, 16-byte aligned); dExtra: [n_rows, K_extra] with row pitch ld_extra, no alignment
+ * needed, 0 <= K_extra <= K.  dY may alias dOut. */
+int b200gnn_relu_dropout_bwd_add_f32(const float* dOut, const float* dExtra, int64_t ld_extra, int64_t K_extra,
+                                     const float* Xout, int64_t n_rows, int64_t K, float p, float* dY, void* stream);
 /* Backward of out = dropout_p(relu(BN_train(Y))): given dOut, out (for the
  * mask: out>0 <=> kept and active), Y and the saved batch mean/invstd, writes
  * dY, dgamma[K], dbeta[K] and (if non-NULL) dbias[K] = column sums of dY.
